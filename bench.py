@@ -188,6 +188,40 @@ def cpu_replay_baseline(stream, payload_bytes, threads, budget_s=20.0, max_passe
                       "reference worker is closed source (README.md:131)"}
 
 
+DUMP_CHUNKS, DUMP_CHUNK_BYTES, DUMP_SEED = 4, 16 << 10, 20240601
+
+
+def save_output(d, name, arr):
+    """One output array as DIR/<name>.npy, in float32 (bytes are 0..255: exact) or float64."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    arr = np.asarray(arr)
+    np.save(os.path.join(d, name + ".npy"), arr.astype(np.float64 if arr.dtype.itemsize > 2 else np.float32))
+
+
+def dump_replay_outputs(d, w, t, nbuf, resp, replays):
+    """What the last replay of the resident trace left for its caller: the response stream of that replay, a
+    digest of every buffer (tfw_dev_digest, as two 32-bit halves) and a fixed, seeded sample of their bytes
+    (DUMP_CHUNKS x DUMP_CHUNK_BYTES per buffer: 64 x 64 KiB = 16 MB as float32 for the default 4 GiB)."""
+    import numpy as np
+    assert len(resp) % replays == 0, (len(resp), replays)
+    per = len(resp) // replays
+    save_output(d, "replay_responses", np.frombuffer(resp[len(resp) - per:], dtype=np.uint8))
+    rng = np.random.default_rng(DUMP_SEED)
+    digests, sample, offsets = [], [], []
+    for h in range(1, nbuf + 1):
+        size, ptr = t.buffer_info(h)
+        dg = w.dev_digest(ptr, size)
+        digests.append((dg >> 32, dg & 0xFFFFFFFF))
+        n = min(DUMP_CHUNK_BYTES, size)
+        offs = np.sort(rng.integers(0, size - n + 1, DUMP_CHUNKS))
+        offsets.append(offs)
+        sample.append(np.concatenate([w.dev_read(ptr + int(o), n) for o in offs]))
+    save_output(d, "replay_buffer_digests", np.array(digests, dtype=np.uint64))
+    save_output(d, "replay_buffer_sample_offsets", np.array(offsets, dtype=np.int64))
+    save_output(d, "replay_buffer_sample", np.stack(sample))
+
+
 def bench_config(args, world):
     """The `config` object of the JSON line -- the same for both arms (the reference arm runs `your arm's config`)."""
     payload = args.copies * args.payload_mib * MIB
@@ -268,7 +302,10 @@ def main():
     ap.add_argument("--no-c4", action="store_true", help="skip the 256 GiB-on-one-GPU policy sweep")
     ap.add_argument("--c5-gib", type=int, default=0, help="size of the C5 vGPU address space (0 = 1 TiB at 8 GPUs, scaled down with fewer)")
     ap.add_argument("--swap-regions", type=int, default=8, help="1 GiB regions evicted/prefetched per GPU in the swap leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed legs computed in their last step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(3, args.warmup)
@@ -323,7 +360,7 @@ def main():
     barrier()
     dev_ms = e0.elapsed_time(e1)
     s1 = w.stats()
-    w.poll()
+    replay_resp = w.poll()   # the responses of every replay since the trace was loaded, each the same length
     launches = sum(s1[k] - s0[k] for k in ("mover_launches", "client_launches", "gate_launches"))
     mover_launches = s1["mover_launches"] - s0["mover_launches"]
     if world > 1:
@@ -339,10 +376,12 @@ def main():
     avg_launch_ms = dev_ms / max(1, mover_launches)
     achieved = algo_per_launch / (avg_launch_ms * 1e-3) / 1e9
     traffic, traffic_note = ncu_traffic()
+    if args.dump_outputs and rank == 0:
+        dump_replay_outputs(args.dump_outputs, w, t, args.buffers, replay_resp, args.warmup + args.steps)
     t.free()
 
     # ---------------- leg 2: end to end from pinned host memory through the C-ABI ----------------
-    e2e_steps = min(args.steps, 10)
+    e2e_steps = args.steps
     tail = bytes(wire.Builder().d2h(1, 0, 4096).sync())
     tail_arr = np.frombuffer(tail, dtype=np.uint8)
     free_all = wire.Builder()
@@ -376,6 +415,8 @@ def main():
         e2e_s = float(tt.item())
     e2e_val = world * payload_per_step * e2e_steps / e2e_s / 1e9
     clocks = sampler.summary()
+    if args.dump_outputs and rank == 0:
+        save_output(args.dump_outputs, "e2e_responses", np.frombuffer(resp, dtype=np.uint8))
     h2d_per_step = (s1["h2d_dma_bytes"] - s0["h2d_dma_bytes"]) // e2e_steps
     d2h_per_step = (s1["d2h_bytes"] - s0["d2h_bytes"]) // e2e_steps
     assert len(resp) >= 4096 and d2h_per_step >= 4096

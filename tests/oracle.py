@@ -128,3 +128,26 @@ def pattern(seed, nbytes):
     out = np.empty(nbytes, dtype=np.uint8)
     lib.tfo_pattern(seed, _P(out.ctypes.data), nbytes)
     return out
+
+
+# ---- what the reference's own C programs printed (tests/golden/reference_runs.json, oracle/record_golden.py) ----
+REF_BUILD = os.path.join(ROOT, "oracle", "_ref")
+
+
+def reference_run(name):
+    """{"returncode", "stdout": [lines]} of one recorded run of the reference's programs."""
+    import json
+    with open(os.path.join(ROOT, "tests", "golden", "reference_runs.json")) as f:
+        return json.load(f)[name]
+
+
+def abi_suite_results(lines):
+    """The assertions of the reference's provider ABI suite output: [(section, message, passed)]."""
+    out, section = [], None
+    for ln in lines:
+        s = ln.strip()
+        if s.startswith("=== Testing ") and s.endswith(" ==="):
+            section = s[len("=== Testing "):-len(" ===")]
+        elif section and s[:2] in ("✓ ", "✗ "):
+            out.append((section, s[2:], s[0] == "✓"))
+    return out

@@ -189,7 +189,7 @@ def test_peer_tier_round_trip(flags):
     """Needs >= 2 GPUs: evict to peer HBM over NVLink (mover kernel / copy engine), read it
     back THROUGH the same vGPU address, prefetch, stripe a batch over all peers."""
     if _ndev() < 2:
-        pytest.skip("needs at least 2 GPUs (run under gpurun --gpus 2)")
+        pytest.skip("needs at least 2 GPUs")
     from tensor_fusion_b200 import vram as V
     peers = list(range(1, _ndev()))
     n = 16
@@ -216,7 +216,7 @@ def test_peer_tier_round_trip(flags):
 
 def test_policy_prefers_peer_hbm_over_host():
     if _ndev() < 2:
-        pytest.skip("needs at least 2 GPUs (run under gpurun --gpus 2)")
+        pytest.skip("needs at least 2 GPUs")
     from tensor_fusion_b200 import vram as V
     peers = list(range(1, _ndev()))
     n, budget = 12, 4

@@ -1,6 +1,6 @@
 """Pins the CPU oracle to every golden vector / known-answer test the reference
 holds for this path (SURVEY.md 8c).  Each test cites the Go test it transliterates.
-Reference root: /root/reference (not needed at run time; values are restated here).
+The reference is not needed at run time: its values are restated here and in tests/golden/.
 """
 import ctypes as C
 import os
@@ -314,18 +314,17 @@ def test_vectors_from_golden_file():
 
 
 def test_reference_c_provider_and_mock_driver_known_answers():
-    """The reference's C half, compiled from its own sources into oracle/_ref (when /root/reference was
-    present at build time): 49/49 ABI assertions, and the mock driver's 100-launches-per-second window."""
+    """The reference's C half as it ran when compiled from its own sources (tests/golden/reference_runs.json):
+    49/49 ABI assertions, and the mock driver's 100-launches-per-second window."""
     import json
-    import subprocess
     g = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "reference_vectors.json")))
-    ref = os.path.join(os.path.dirname(os.path.dirname(__file__)), "oracle", "_ref")
-    if not os.path.exists(os.path.join(ref, "test_accelerator_ref")):
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
-    r = subprocess.run([os.path.join(ref, "test_accelerator_ref")], capture_output=True, text=True, cwd=ref, timeout=120)
-    passed = int(r.stdout.split("Passed:")[1].split()[0])
-    assert r.returncode == 0 and "Failed:       0" in r.stdout and passed >= g["provider_stub"]["assertions"]   # +3 when a mock process is registered
-    r = subprocess.run([os.path.join(ref, "test_rate_limit")], capture_output=True, text=True, cwd=ref, timeout=120)
-    assert r.returncode == 0, r.stdout[-500:]
-    assert f"Successful launches: {g['mock_rate_limit']['accepted']}" in r.stdout
-    assert f"Blocked launches: {g['mock_rate_limit']['launches'] - g['mock_rate_limit']['accepted']}" in r.stdout
+    r = oracle.reference_run("abi_suite")
+    out = "\n".join(r["stdout"])
+    passed = int(out.split("Passed:")[1].split()[0])
+    assert r["returncode"] == 0 and "Failed:       0" in out and passed >= g["provider_stub"]["assertions"]   # +3 when a mock process is registered
+    assert len(oracle.abi_suite_results(r["stdout"])) == passed
+    r = oracle.reference_run("mock_rate_limit")
+    out = "\n".join(r["stdout"])
+    assert r["returncode"] == 0, out[-500:]
+    assert f"Successful launches: {g['mock_rate_limit']['accepted']}" in out
+    assert f"Blocked launches: {g['mock_rate_limit']['launches'] - g['mock_rate_limit']['accepted']}" in out
