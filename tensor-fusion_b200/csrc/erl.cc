@@ -129,15 +129,4 @@ double tick(tfq::QuotaFile& q, uint32_t idx, State& st, const Config& cfg, uint3
   return rebalance(q, idx, now_secs, st.current_rate, capacity, target, st.smoothed_util);
 }
 
-uint32_t up_limit_percent(int64_t compute_percent, double tflops_limit, double max_tflops) {
-  if (compute_percent > 0) return (uint32_t)compute_percent;
-  if (tflops_limit > 0 && max_tflops > 0) {
-    const double pct = std::ceil(tflops_limit / max_tflops * 100.0);
-    if (pct < 1) return 1;
-    if (pct > 100) return 100;
-    return (uint32_t)pct;
-  }
-  return 100;
-}
-
 }  // namespace tferl

@@ -9,6 +9,7 @@
 #pragma once
 #include <stdint.h>
 
+#include <cmath>
 #include <string>
 
 #include "shm_quota.h"
@@ -45,6 +46,16 @@ double rebalance(tfq::QuotaFile& q, uint32_t idx, double now_secs, double rate, 
 // Returns the token balance after the step.
 double tick(tfq::QuotaFile& q, uint32_t idx, State& st, const Config& cfg, uint32_t up_limit,
             double util_percent, double now_secs);                                               // :412-446
-uint32_t up_limit_percent(int64_t compute_percent, double tflops_limit, double max_tflops);     // controller.go:307-325
+// controller.go:307-325.  Inline: the worker executable uses it without linking the controller (and QuotaFile).
+inline uint32_t up_limit_percent(int64_t compute_percent, double tflops_limit, double max_tflops) {
+  if (compute_percent > 0) return (uint32_t)compute_percent;
+  if (tflops_limit > 0 && max_tflops > 0) {
+    const double pct = std::ceil(tflops_limit / max_tflops * 100.0);
+    if (pct < 1) return 1;
+    if (pct > 100) return 100;
+    return (uint32_t)pct;
+  }
+  return 100;
+}
 
 }  // namespace tferl

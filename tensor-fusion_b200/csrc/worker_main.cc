@@ -19,7 +19,6 @@
 
 #include <atomic>
 #include <cerrno>
-#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -29,6 +28,7 @@
 #include <thread>
 #include <vector>
 
+#include "erl.h"
 #include "hv_handshake.h"
 #include "tfw_shm_ring.h"
 #include "tfw_wire.h"
@@ -73,20 +73,6 @@ uint64_t g_vram_limit_from_hypervisor = 0;
 uint32_t g_sm_percent_from_hypervisor = 0;  // hard isolation: computeUpLimit(tflops_limit / the GPU's max TFLOPS)
 long g_auto_freeze_ttl_ms = 0;  // auto_freeze.freeze_to_mem_ttl of the hypervisor's pod info, or $TF_AUTO_FREEZE_TTL_MS
 
-// Idle policy of one session: a vGPU whose client has been silent for the TTL gives its HBM back (freeze to
-// memory); the client's next byte brings it back before anything is executed.
-struct IdlePolicy {
-  timespec last{};
-  IdlePolicy() { clock_gettime(CLOCK_MONOTONIC, &last); }
-  void activity() { clock_gettime(CLOCK_MONOTONIC, &last); }
-  bool due() const {
-    if (g_auto_freeze_ttl_ms <= 0) return false;
-    timespec now;
-    clock_gettime(CLOCK_MONOTONIC, &now);
-    return (now.tv_sec - last.tv_sec) * 1000 + (now.tv_nsec - last.tv_nsec) / 1000000 >= g_auto_freeze_ttl_ms;
-  }
-};
-
 void hypervisor_handshake() {
   const tfhv::Result r = tfhv::handshake("tensorfusion-worker");  // pkg/constants/env.go:61
   if (!getenv("HYPERVISOR_IP")) return;
@@ -95,12 +81,11 @@ void hypervisor_handshake() {
   g_vram_limit_from_hypervisor = r.vram_limit;
   if (r.auto_freeze_ttl_ms > 0 && !getenv("TF_AUTO_FREEZE_TTL_MS")) g_auto_freeze_ttl_ms = r.auto_freeze_ttl_ms;
   // hard isolation without an explicit SM limit from the operator: the share of the GPU the pod's TFLOPS limit
-  // buys (computeUpLimit, controller.go:307-325; B200 = 2250 dense bf16 TFLOPS, gpu-public-gpu-info.yaml:380-385)
+  // buys (B200 = 2250 dense bf16 TFLOPS, gpu-public-gpu-info.yaml:380-385)
   if (r.hard_isolation && r.tflops_limit > 0) {
     const char* mt = getenv("TF_GPU_MAX_TFLOPS");
     const double max_tflops = mt && atof(mt) > 0 ? atof(mt) : 2250.0;
-    const double pct = std::ceil(r.tflops_limit / max_tflops * 100.0);
-    g_sm_percent_from_hypervisor = pct < 1 ? 1 : pct > 100 ? 100 : (uint32_t)pct;
+    g_sm_percent_from_hypervisor = tferl::up_limit_percent(0, r.tflops_limit, max_tflops);
   }
   logf("pod info: vram_limit=%llu tflops_limit=%g isolation=%s auto_freeze_ttl_ms=%ld sm_percent=%u", (unsigned long long)r.vram_limit, r.tflops_limit,
        r.hard_isolation ? "hard" : "soft", r.auto_freeze_ttl_ms, g_sm_percent_from_hypervisor);
@@ -130,8 +115,103 @@ tfw_worker* make_worker(int device) {
   return w;
 }
 
-void serve_shm_session(tfsr_header* hdr, uint8_t* base, uint64_t total_bytes, int device, uint32_t session, int lock_fd, const std::string& ring_path,
-                       tfw_worker* ready = nullptr);
+// What every session does, whatever the transport: the vGPU's control words and idle policy, submitting around a full
+// response arena or ring, the window of spans whose DMA may still read client bytes, and the close-out.  The transports
+// keep how bytes arrive, how responses leave and how the client's end is seen.
+struct Session {
+  struct Span { uint64_t ticket, upto; };
+  tfw_worker* w;
+  uint64_t* released = nullptr;  // where the end of a span is published once its DMA has completed (the rings' c2w_tail)
+  std::deque<Span> inflight;     // oldest first
+  timespec active{};             // the client's last activity, where the freeze-to-memory TTL starts
+  uint64_t bytes_in = 0;
+
+  Session(tfw_worker* worker, uint64_t* released_to = nullptr) : w(worker), released(released_to) { touch(); }
+  void touch() { clock_gettime(CLOCK_MONOTONIC, &active); }
+  // The provider's control words (AccelSnapshot / AccelResume / hard limits, DESIGN §7c): 0 running, 1 frozen by the
+  // provider (nothing is read, so the client is back-pressured; responses keep leaving), 2 frozen by the idle policy.
+  int control() { int frozen = 0; tfw_worker_poll_control(w, &frozen); return frozen; }
+  // The client has sent bytes: a vGPU the idle policy froze comes back before any of them executes.  False while the HBM
+  // is not available yet.
+  bool thaw(int frozen) {
+    if (frozen == 2 && tfw_worker_auto_resume(w) != TFW_OK) { usleep(2000); return false; }
+    touch();
+    return true;
+  }
+  // The client is quiet and the vGPU runs: once the TTL has passed it gives its HBM back (true), and the TTL starts over.
+  bool freeze_if_idle() {
+    if (g_auto_freeze_ttl_ms <= 0) return false;
+    timespec now;
+    clock_gettime(CLOCK_MONOTONIC, &now);
+    if ((now.tv_sec - active.tv_sec) * 1000 + (now.tv_nsec - active.tv_nsec) / 1000000 < g_auto_freeze_ttl_ms) return false;
+    uint64_t moved = 0;
+    if (tfw_worker_auto_freeze(w, &moved) == TFW_OK) logf("idle for %ld ms: vGPU frozen to memory (%llu bytes)", g_auto_freeze_ttl_ms, (unsigned long long)moved);
+    touch();
+    return true;
+  }
+  // tfw_submit until the parser has taken what it can.  TFW_ERR_EXHAUSTED (the response arena or ring is full) calls
+  // make_room(), then the frame is resumed where the parser stopped; make_room() false ends the attempt.
+  template <class MakeRoom>
+  tfw_status submit(const uint8_t* p, size_t n, size_t* used, MakeRoom make_room) {
+    *used = 0;
+    for (;;) {
+      size_t u = 0;
+      const tfw_status rc = tfw_submit(w, p + *used, n - *used, &u);
+      *used += u;
+      if (rc != TFW_ERR_EXHAUSTED) return rc;
+      if (!make_room()) return TFW_ERR_FAILED;
+    }
+  }
+  // Fence what has been submitted; past `window` spans in flight, wait for the oldest.
+  bool fence(size_t window, uint64_t upto = 0) {
+    uint64_t ticket = 0;
+    if (tfw_fence(w, &ticket) != TFW_OK) return false;
+    inflight.push_back({ticket, upto});
+    return inflight.size() <= window || retire(true);
+  }
+  // Release the leading spans whose DMA has completed; `block` waits for the first.
+  bool retire(bool block) {
+    while (!inflight.empty()) {
+      int done = 0;
+      if (block) { if (tfw_fence_wait(w, inflight.front().ticket) != TFW_OK) return false; done = 1; }
+      else if (tfw_fence_query(w, inflight.front().ticket, &done) != TFW_OK) return false;
+      if (!done) break;
+      if (released) __atomic_store_n(released, inflight.front().upto, __ATOMIC_RELEASE);
+      inflight.pop_front();
+      block = false;
+    }
+    return true;
+  }
+  // Unless the session failed, everything submitted executes and deliver() hands out what it produced; then the session's
+  // log line, and the vGPU goes.
+  template <class Deliver>
+  void end(bool failed, Deliver deliver) {
+    if (!failed) {
+      tfw_flush(w);
+      retire(true);
+      deliver();
+    }
+    tfw_stats st{};
+    tfw_get_stats(w, &st);
+    logf("session closed: %llu bytes in, %llu frames, %llu payload bytes, %llu mover launches", (unsigned long long)bytes_in,
+         (unsigned long long)st.frames, (unsigned long long)st.payload_bytes, (unsigned long long)st.mover_launches);
+    tfw_worker_destroy(w);
+  }
+};
+
+// A fresh header for rings of `total` bytes, published to clients last (magic, then worker_ready).
+void init_ring_header(tfsr_header* hdr, uint64_t total) {
+  std::memset(hdr, 0, sizeof *hdr);
+  hdr->version = TFSR_VERSION;
+  hdr->total_bytes = total;
+  tfsr_layout(total, &hdr->c2w_off, &hdr->c2w_size, &hdr->w2c_off, &hdr->w2c_size);
+  hdr->worker_pid = (uint32_t)getpid();
+  hdr->session = 1;
+  __atomic_store_n(&hdr->magic, TFSR_MAGIC, __ATOMIC_RELEASE);
+  __atomic_store_n(&hdr->worker_ready, 1u, __ATOMIC_RELEASE);
+}
+
+void serve_rings(tfsr_header* hdr, uint8_t* base, uint64_t total_bytes, uint32_t session, int lock_fd, const std::string& ring_path, tfw_worker* w);
 
 bool recv_exact(int fd, void* p, size_t n, int timeout_ms) {
   uint8_t* b = static_cast<uint8_t*>(p);
@@ -152,7 +232,7 @@ bool recv_exact(int fd, void* p, size_t n, int timeout_ms) {
 // TFCS_OP_UPGRADE_SHM: a client on this node asks to continue on shared-memory rings it has created.  Returns true if
 // the session was served (on the rings); false = stay on the socket (the refusal has been sent).
 // `w`: the session's worker, created before the first frame was read; when this returns true the rings' session has used and destroyed it
-bool try_upgrade_to_shm(int fd, int device, const tfcs_frame_hdr& h, const std::string& name, tfw_worker* w) {
+bool try_upgrade_to_shm(int fd, const tfcs_frame_hdr& h, const std::string& name, tfw_worker* w) {
   auto refuse = [&](uint32_t code) {
     tfcs_frame_hdr r = h;
     r.opcode = TFCS_OP_RESP_ERROR;
@@ -176,14 +256,7 @@ bool try_upgrade_to_shm(int fd, int device, const tfcs_frame_hdr& h, const std::
   if (m == MAP_FAILED) { close(sfd); return refuse(TFW_ERR_EXHAUSTED); }
   if (tfw_host_register(m, total) != TFW_OK) { munmap(m, total); close(sfd); return refuse(TFW_ERR_EXHAUSTED); }
   tfsr_header* hdr = static_cast<tfsr_header*>(m);
-  std::memset(hdr, 0, sizeof *hdr);
-  hdr->version = TFSR_VERSION;
-  hdr->total_bytes = total;
-  tfsr_layout(total, &hdr->c2w_off, &hdr->c2w_size, &hdr->w2c_off, &hdr->w2c_size);
-  hdr->worker_pid = (uint32_t)getpid();
-  hdr->session = 1;
-  __atomic_store_n(&hdr->magic, TFSR_MAGIC, __ATOMIC_RELEASE);
-  __atomic_store_n(&hdr->worker_ready, 1u, __ATOMIC_RELEASE);
+  init_ring_header(hdr, total);
   tfcs_frame_hdr r = h;
   r.opcode = TFCS_OP_RESP_ACK;
   r.length = 0;
@@ -192,7 +265,7 @@ bool try_upgrade_to_shm(int fd, int device, const tfcs_frame_hdr& h, const std::
   ok = ok && __atomic_load_n(&hdr->client_pid, __ATOMIC_ACQUIRE) != 0;
   if (ok) {
     logf("connection upgraded to shared-memory rings %s (%llu MiB)", path.c_str(), (unsigned long long)(total >> 20));
-    serve_shm_session(hdr, static_cast<uint8_t*>(m), total, device, 1, sfd, path, w);
+    serve_rings(hdr, static_cast<uint8_t*>(m), total, 1, sfd, path, w);
   }  // (else: the client never attached; the caller keeps the worker and finds the socket dead)
   __atomic_store_n(&hdr->worker_ready, 0u, __ATOMIC_RELEASE);
   tfw_host_unregister(m);
@@ -202,6 +275,8 @@ bool try_upgrade_to_shm(int fd, int device, const tfcs_frame_hdr& h, const std::
   return ok;
 }
 
+// One TCP connection: bytes are received into two pinned rings, responses go back on the socket; recv() <= 0 is the
+// client's end.
 void serve(int fd, int device) {
   int one = 1;
   setsockopt(fd, IPPROTO_TCP, TCP_NODELAY, &one, sizeof one);
@@ -216,12 +291,11 @@ void serve(int fd, int device) {
     return;
   }
   // A client on this node may propose shared-memory rings with its very first frame (TFCS_OP_UPGRADE_SHM).
-  tfcs_frame_hdr first{};
-  size_t carried = 0;  // bytes of the stream already taken off the socket (a first frame that was no upgrade)
   {
     uint8_t peek[TFCS_HDR_BYTES];
     ssize_t k;
     do { k = recv(fd, peek, sizeof peek, MSG_PEEK | MSG_WAITALL); } while (k < 0 && errno == EINTR);
+    tfcs_frame_hdr first{};
     if (k == (ssize_t)sizeof peek) {
       std::memcpy(&first, peek, sizeof first);
       if (first.magic == TFCS_MAGIC && first.opcode == TFCS_OP_UPGRADE_SHM && first.length <= 255) {
@@ -229,16 +303,13 @@ void serve(int fd, int device) {
         uint8_t skip[TFCS_HDR_BYTES];
         if (!recv_exact(fd, skip, sizeof skip, 5000) || !recv_exact(fd, name, (size_t)tfcs_pad16(first.length), 5000)) { tfw_worker_destroy(w); close(fd); return; }
         name[first.length] = 0;
-        if (try_upgrade_to_shm(fd, device, first, name, w)) { close(fd); return; }  // (the rings' session took the worker)
+        if (try_upgrade_to_shm(fd, first, name, w)) { close(fd); return; }  // (the rings' session took the worker)
       }
     }
-    (void)carried;
   }
-  tfw_status rc = TFW_OK;
   // Two pinned rings: while the GPU still reads ring A (in-place DMA), the socket fills ring B.
   const size_t ring = 64u << 20;
   uint8_t* bufs[2] = {nullptr, nullptr};
-  uint64_t tickets[2] = {0, 0};
   std::vector<uint8_t> out(16u << 20);
   if (tfw_host_alloc(ring, reinterpret_cast<void**>(&bufs[0])) != TFW_OK || tfw_host_alloc(ring, reinterpret_cast<void**>(&bufs[1])) != TFW_OK) {
     if (bufs[0]) tfw_host_free(bufs[0]);
@@ -246,10 +317,9 @@ void serve(int fd, int device) {
     close(fd);
     return;
   }
+  Session s(w);
   int cur = 0;
   size_t fill = 0;
-  uint64_t total = 0;
-  IdlePolicy idle;
   auto drain = [&](bool block) {
     for (;;) {
       size_t m = 0;
@@ -259,29 +329,21 @@ void serve(int fd, int device) {
     }
   };
   for (;;) {
-    uint8_t* buf = bufs[cur];
-    // AccelSnapshot / AccelResume of the provider arrive through the stats record.  A frozen vGPU stops
-    // reading its socket, so the client is back-pressured by TCP until the resume.
-    if (g_stop.load()) break;  // SIGTERM: finish what was submitted (flush + drain below) and close
-    int frozen = 0;
-    tfw_worker_poll_control(w, &frozen);
-    if (frozen == 1) {  // frozen by the provider: the socket is not read, the client is back-pressured
-      if (!drain(false)) break;
-      usleep(2000);
-      continue;
-    }
+    if (g_stop.load()) break;  // SIGTERM: finish what was submitted (the close-out below) and close
+    const int frozen = s.control();
+    if (frozen == 1) { if (!drain(false)) break; usleep(2000); continue; }  // the client is back-pressured by TCP
     // Responses (D2H payloads, SYNC acks) become ready asynchronously: while the client is quiet,
     // keep delivering them instead of blocking in recv().
     pollfd pf{fd, POLLIN, 0};
-    int pr = poll(&pf, 1, 2);
+    const int pr = poll(&pf, 1, 2);
     if (pr == 0) {
       if (!drain(false)) break;
-      if (!frozen && idle.due()) { uint64_t moved = 0; if (tfw_worker_auto_freeze(w, &moved) == TFW_OK) logf("idle for %ld ms: vGPU frozen to memory (%llu bytes)", g_auto_freeze_ttl_ms, (unsigned long long)moved); }
+      if (!frozen) s.freeze_if_idle();
       continue;
     }
     if (pr < 0 && errno == EINTR) continue;
-    idle.activity();
-    if (frozen == 2 && tfw_worker_auto_resume(w) != TFW_OK) { usleep(2000); continue; }  // HBM not available yet: try again
+    if (!s.thaw(frozen)) continue;
+    uint8_t* buf = bufs[cur];
     ssize_t n = recv(fd, buf + fill, ring - fill, 0);
     if (n < 0 && errno == EINTR) continue;
     if (n <= 0) break;
@@ -292,40 +354,28 @@ void serve(int fd, int device) {
       if (k <= 0) break;
       n += k;
     }
-    total += (uint64_t)n;
-    size_t have = fill + (size_t)n, used = 0;
-    for (;;) {
-      rc = tfw_submit(w, buf, have, &used);
-      if (rc != TFW_ERR_EXHAUSTED) break;  // response arena full: ship responses, then resume where we stopped
-      tfw_flush(w);
-      if (!drain(true)) { rc = TFW_ERR_FAILED; break; }
-      std::memmove(buf, buf + used, have - used);
-      have -= used;
-    }
+    s.bytes_in += (uint64_t)n;
+    const size_t have = fill + (size_t)n;
+    size_t used = 0;
+    // response arena full: ship responses, then resume where the parser stopped
+    const tfw_status rc = s.submit(buf, have, &used, [&] { tfw_flush(w); return drain(true); });
     if (rc != TFW_OK) { logf("submit failed: %d (%s)", rc, tfw_last_error(w)); break; }
-    if (tfw_fence(w, &tickets[cur]) != TFW_OK) break;
-    const int nxt = cur ^ 1;
-    if (tickets[nxt] && tfw_fence_wait(w, tickets[nxt]) != TFW_OK) break;  // the other ring is free again
-    const size_t rest = have - used;  // < 64 bytes: a partial header, carried over to the other ring
-    std::memcpy(bufs[nxt], buf + used, rest);
-    fill = rest;
-    cur = nxt;
+    if (!s.fence(1)) break;  // one span in flight: the other ring, refilled next, has been read by the GPU
+    cur ^= 1;
+    fill = have - used;  // < 64 bytes: a partial header, moved to the front of the other ring
+    std::memcpy(bufs[cur], buf + used, fill);
     if (!drain(false)) break;
   }
-  tfw_flush(w);
-  drain(true);
-  tfw_stats st{};
-  tfw_get_stats(w, &st);
-  logf("session closed: %llu bytes in, %llu frames, %llu payload bytes, %llu mover launches", (unsigned long long)total,
-       (unsigned long long)st.frames, (unsigned long long)st.payload_bytes, (unsigned long long)st.mover_launches);
+  s.end(false, [&] { drain(true); });
   tfw_host_free(bufs[0]);
   tfw_host_free(bufs[1]);
-  tfw_worker_destroy(w);
   close(fd);
 }
 
 // ---- shared-memory transport (include/tfw_shm_ring.h) -----------------------------------------------------
-struct Idle {  // spin, then 20 us naps, then 200 us naps once the client has been quiet for ~10 ms
+// How the worker waits for the client on the rings: spin, then 20 us naps, then 200 us naps once the client has been
+// quiet for ~10 ms.
+struct Backoff {
   int n = 0;
   void reset() { n = 0; }
   void pause() {
@@ -334,11 +384,13 @@ struct Idle {  // spin, then 20 us naps, then 200 us naps once the client has be
     timespec ts{0, n < 2500 ? 20000 : 200000};
     nanosleep(&ts, nullptr);
   }
+  bool probe_due() const { return n >= 5000 && n % 5000 == 0; }  // 5000 naps of 200 us = 1 s: time to probe the client's liveness
 };
 
-void serve_shm_session(tfsr_header* hdr, uint8_t* base, uint64_t total_bytes, int device, uint32_t session, int lock_fd, const std::string& ring_path,
-                       tfw_worker* ready) {
-  tfw_worker* w = ready ? ready : make_worker(device);
+// One client session on the rings; `w` (may be null: worker_closed at once) is the session's vGPU and is destroyed here.
+// Bytes are read in place from the client -> worker ring; responses are produced into the worker -> client ring by the
+// library (the response sink); the client ends the session with client_closed, or is found gone through its liveness lock.
+void serve_rings(tfsr_header* hdr, uint8_t* base, uint64_t total_bytes, uint32_t session, int lock_fd, const std::string& ring_path, tfw_worker* w) {
   if (!w) {
     __atomic_store_n(&hdr->worker_closed, session, __ATOMIC_RELEASE);
     return;
@@ -348,38 +400,20 @@ void serve_shm_session(tfsr_header* hdr, uint8_t* base, uint64_t total_bytes, in
   uint64_t c2w_off = 0, up = 0, w2c_off = 0, down = 0;
   tfsr_layout(total_bytes, &c2w_off, &up, &w2c_off, &down);
   uint8_t* c2w = base + c2w_off;
-  uint8_t* w2c = base + w2c_off;
-  uint64_t rd = hdr->c2w_tail;          // read cursor; the shared tail trails it until the DMA of a span is done
   // Responses are produced in the worker -> client ring itself: D2H payloads are written there by the copy
   // engine (the mapping is page-locked), the head cursor moves when the GPU is done with a piece.
-  tfw_response_sink sink{};
-  sink.struct_size = sizeof sink;
-  sink.ring = w2c;
-  sink.ring_bytes = down;
-  sink.head = &hdr->w2c_head;
-  sink.tail = &hdr->w2c_tail;
-  const bool direct = !getenv("TFW_SHM_NO_SINK") && tfw_set_response_sink(w, &sink) == TFW_OK;
+  const tfw_response_sink sink{sizeof(tfw_response_sink), 0, base + w2c_off, down, &hdr->w2c_head, &hdr->w2c_tail};
+  if (tfw_set_response_sink(w, &sink) != TFW_OK) {
+    fprintf(stderr, "[tensor-fusion-worker] session %u: no response sink on the rings: %s\n", session, tfw_last_error(w));
+    tfw_worker_destroy(w);
+    __atomic_store_n(&hdr->worker_closed, session, __ATOMIC_RELEASE);
+    return;
+  }
+  Session s(w, &hdr->c2w_tail);
+  uint64_t rd = hdr->c2w_tail;  // read cursor; the shared tail trails it until the DMA of a span is done
   uint64_t wr = hdr->w2c_head;
-  struct Span { uint64_t ticket, upto; };
-  std::deque<Span> inflight;
-  alignas(16) uint8_t joined[TFCS_HDR_BYTES];
-  uint64_t total = 0;
-  Idle idle;
-  IdlePolicy idle_policy;
-  bool failed = false;
-
-  auto release_done = [&](bool block) {
-    while (!inflight.empty()) {
-      int done = 0;
-      if (block) { if (tfw_fence_wait(w, inflight.front().ticket) != TFW_OK) return false; done = 1; }
-      else if (tfw_fence_query(w, inflight.front().ticket, &done) != TFW_OK) return false;
-      if (!done) break;
-      __atomic_store_n(&hdr->c2w_tail, inflight.front().upto, __ATOMIC_RELEASE);
-      inflight.pop_front();
-      block = false;
-    }
-    return true;
-  };
+  bool ring_full = false;
+  auto closed = [&] { return __atomic_load_n(&hdr->client_closed, __ATOMIC_ACQUIRE) >= session; };
   // a client that died without saying so (include/tfw_shm_ring.h: liveness lock); probed once a second while silent
   auto client_gone = [&]() {
 #ifdef TFSR_HAVE_LIVENESS
@@ -389,147 +423,95 @@ void serve_shm_session(tfsr_header* hdr, uint8_t* base, uint64_t total_bytes, in
     return false;
 #endif
   };
-
-  // responses go straight into the worker -> client ring; returns bytes moved, -1 on error
-  bool ring_full = false;
-  auto pump_responses = [&]() -> long {
-    long moved = 0;
-    if (direct) {
-      size_t m = 0;
-      if (tfw_poll_responses(w, nullptr, 0, &m) != TFW_OK) return -1;
-      const uint64_t head = __atomic_load_n(&hdr->w2c_head, __ATOMIC_RELAXED);
-      moved = (long)(head - wr);
-      wr = head;
-      ring_full = down - (head - __atomic_load_n(&hdr->w2c_tail, __ATOMIC_ACQUIRE)) < (1u << 20);
-      return moved;
-    }
-    for (;;) {
-      const uint64_t tail = __atomic_load_n(&hdr->w2c_tail, __ATOMIC_ACQUIRE);
-      const uint64_t free_b = down - (wr - tail);
-      ring_full = free_b == 0;
-      if (ring_full) return moved;
-      const uint64_t pos = wr % down;
-      size_t m = 0;
-      // publish in pieces of 4 MiB: the client copies piece k out while piece k+1 is being written
-      const uint64_t cap = std::min<uint64_t>(std::min<uint64_t>(free_b, down - pos), 4u << 20);
-      if (tfw_poll_responses(w, w2c + pos, (size_t)cap, &m) != TFW_OK) return -1;
-      if (!m) return moved;
-      wr += m;
-      __atomic_store_n(&hdr->w2c_head, wr, __ATOMIC_RELEASE);
-      moved += (long)m;
-    }
+  // publish the responses whose GPU work has completed; returns bytes published, -1 on error
+  auto publish = [&]() -> long {
+    size_t m = 0;
+    if (tfw_poll_responses(w, nullptr, 0, &m) != TFW_OK) return -1;
+    const uint64_t head = __atomic_load_n(&hdr->w2c_head, __ATOMIC_RELAXED);
+    const long moved = (long)(head - wr);
+    wr = head;
+    ring_full = down - (head - __atomic_load_n(&hdr->w2c_tail, __ATOMIC_ACQUIRE)) < (1u << 20);
+    return moved;
   };
-  auto submit_span = [&](const uint8_t* p, size_t n, size_t* used) {
-    *used = 0;
-    for (;;) {
-      size_t u = 0;
-      const tfw_status rc = tfw_submit(w, p + *used, n - *used, &u);
-      *used += u;
-      if (rc != TFW_ERR_EXHAUSTED) return rc;
-      if (direct) {  // the ring is full: publish what completes and wait for the client to consume, then resume the frame
-        Idle wait;
-        const uint64_t tail0 = __atomic_load_n(&hdr->w2c_tail, __ATOMIC_ACQUIRE);
-        while (__atomic_load_n(&hdr->w2c_tail, __ATOMIC_ACQUIRE) == tail0) {
-          if (pump_responses() < 0) return TFW_ERR_FAILED;
-          if (__atomic_load_n(&hdr->client_closed, __ATOMIC_ACQUIRE) >= session || g_stop.load()) return TFW_ERR_FAILED;  // nobody reads any more
-          if (wait.n >= 5000 && wait.n % 5000 == 0 && client_gone()) return TFW_ERR_FAILED;
-          wait.pause();
-        }
-        continue;
-      }
-      tfw_flush(w);  // response arena full: ship what is ready, then resume where the parser stopped
-      Idle wait;
-      while (pump_responses() == 0) {
-        if (__atomic_load_n(&hdr->client_closed, __ATOMIC_ACQUIRE) >= session) return TFW_ERR_FAILED;  // nobody reads any more
-        wait.pause();
-      }
+  // the ring is full: publish what completes and wait for the client to consume, then the frame resumes
+  auto make_room = [&]() {
+    Backoff wait;
+    const uint64_t tail0 = __atomic_load_n(&hdr->w2c_tail, __ATOMIC_ACQUIRE);
+    while (__atomic_load_n(&hdr->w2c_tail, __ATOMIC_ACQUIRE) == tail0) {
+      if (publish() < 0) return false;
+      if (closed() || g_stop.load()) return false;  // nobody reads any more
+      if (wait.probe_due() && client_gone()) return false;
+      wait.pause();
     }
+    return true;
   };
+  alignas(16) uint8_t joined[TFCS_HDR_BYTES];
+  Backoff idle;
+  bool failed = false;
 
   for (;;) {
     if (g_stop.load()) break;  // SIGTERM: drain below, then worker_closed tells the client
-    int frozen = 0;
-    tfw_worker_poll_control(w, &frozen);  // AccelSnapshot / AccelResume (see serve())
-    if (frozen == 1) {
-      pump_responses();
-      usleep(2000);
-      continue;
-    }
-    if (frozen == 2) {  // frozen by the idle policy: the client's next byte brings the vGPU back
+    const int frozen = s.control();
+    if (frozen == 1) { publish(); usleep(2000); continue; }
+    if (frozen == 2) {
       if (__atomic_load_n(&hdr->c2w_head, __ATOMIC_ACQUIRE) == rd) {
-        if (__atomic_load_n(&hdr->client_closed, __ATOMIC_ACQUIRE) >= session) break;
+        if (closed()) break;
         usleep(1000);
         continue;
       }
-      if (tfw_worker_auto_resume(w) != TFW_OK) { usleep(2000); continue; }
-      idle_policy.activity();
+      if (!s.thaw(frozen)) continue;
     }
     bool progress = false;
-    if (!inflight.empty()) {
-      const size_t before = inflight.size();
-      if (!release_done(false)) { failed = true; break; }
-      progress |= inflight.size() != before;
+    if (!s.inflight.empty()) {
+      const size_t before = s.inflight.size();
+      if (!s.retire(false)) { failed = true; break; }
+      progress |= s.inflight.size() != before;
     }
-    const uint64_t head = __atomic_load_n(&hdr->c2w_head, __ATOMIC_ACQUIRE);
-    const uint64_t avail = head - rd;
+    const uint64_t avail = __atomic_load_n(&hdr->c2w_head, __ATOMIC_ACQUIRE) - rd;
     if (avail) {
       const uint64_t pos = rd % up;
       const uint64_t span = std::min<uint64_t>(std::min<uint64_t>(avail, up - pos), 64u << 20);
       size_t used = 0;
-      tfw_status rc = submit_span(c2w + pos, (size_t)span, &used);
+      tfw_status rc = s.submit(c2w + pos, (size_t)span, &used, make_room);
       if (rc != TFW_OK) { logf("submit failed: %d (%s)", rc, tfw_last_error(w)); failed = true; break; }
-      rd += used;
-      total += used;
       const uint64_t rest = span - used;  // < 64 bytes: the front of a header whose tail is not here yet ...
       if (rest && pos + span == up && avail - used >= TFCS_HDR_BYTES) {  // ... or wraps to the start of the ring
         std::memcpy(joined, c2w + pos + used, rest);
         std::memcpy(joined + rest, c2w, TFCS_HDR_BYTES - rest);
         size_t u2 = 0;
-        rc = submit_span(joined, TFCS_HDR_BYTES, &u2);
+        rc = s.submit(joined, TFCS_HDR_BYTES, &u2, make_room);
         if (rc != TFW_OK || u2 != TFCS_HDR_BYTES) { logf("submit (wrapped header) failed: %d (%s)", rc, tfw_last_error(w)); failed = true; break; }
-        rd += TFCS_HDR_BYTES;
-        total += TFCS_HDR_BYTES;
         used += TFCS_HDR_BYTES;
       }
+      rd += used;
+      s.bytes_in += used;
       if (used) {
         progress = true;
-        uint64_t ticket = 0;
-        if (tfw_fence(w, &ticket) != TFW_OK) { failed = true; break; }
-        inflight.push_back({ticket, rd});
-        if (inflight.size() > 6 && !release_done(true)) { failed = true; break; }  // the fence ring holds 8
+        if (!s.fence(6, rd)) { failed = true; break; }  // the fence ring holds 8
       }
     }
-    const long moved = pump_responses();
+    const long moved = publish();
     if (moved < 0) { failed = true; break; }
     progress |= moved > 0;
-    if (!avail && __atomic_load_n(&hdr->client_closed, __ATOMIC_ACQUIRE) >= session &&
-        __atomic_load_n(&hdr->c2w_head, __ATOMIC_ACQUIRE) == rd)
-      break;  // the client is done and everything it wrote has been consumed
-    if (progress) { idle.reset(); idle_policy.activity(); }
+    if (!avail && closed() && __atomic_load_n(&hdr->c2w_head, __ATOMIC_ACQUIRE) == rd) break;  // the client is done and everything it wrote has been consumed
+    if (progress) { idle.reset(); s.touch(); }
     else {
-      if (idle_policy.due() && inflight.empty()) {
-        uint64_t moved = 0;
-        if (tfw_worker_auto_freeze(w, &moved) == TFW_OK) logf("idle for %ld ms: vGPU frozen to memory (%llu bytes)", g_auto_freeze_ttl_ms, (unsigned long long)moved);
-        idle_policy.activity();
-        continue;
-      }
+      if (s.inflight.empty() && s.freeze_if_idle()) continue;
       idle.pause();
-      if (idle.n >= 5000 && idle.n % 5000 == 0 && client_gone()) {  // 5000 naps of 200 us = 1 s
+      if (idle.probe_due() && client_gone()) {
         logf("client of session %u is gone without closing: ending the session", session);
         break;
       }
     }
   }
-  if (!failed) {
-    tfw_flush(w);
-    release_done(true);
+  s.end(failed, [&] {
     // everything is ready after the flush; deliver it.  tfc_close keeps reading until worker_closed, a client
     // that died does not: give up after 2 s without progress.
-    Idle wait;
+    Backoff wait;
     timespec last;
     clock_gettime(CLOCK_MONOTONIC, &last);
     for (;;) {
-      const long m = pump_responses();
+      const long m = publish();
       if (m < 0 || !ring_full) break;
       timespec now;
       clock_gettime(CLOCK_MONOTONIC, &now);
@@ -537,13 +519,8 @@ void serve_shm_session(tfsr_header* hdr, uint8_t* base, uint64_t total_bytes, in
       else if (now.tv_sec - last.tv_sec >= 2) break;
       wait.pause();
     }
-  }
+  });
   __atomic_store_n(&hdr->c2w_tail, rd, __ATOMIC_RELEASE);
-  tfw_stats st{};
-  tfw_get_stats(w, &st);
-  logf("session closed: %llu bytes in, %llu frames, %llu payload bytes, %llu mover launches", (unsigned long long)total,
-       (unsigned long long)st.frames, (unsigned long long)st.payload_bytes, (unsigned long long)st.mover_launches);
-  tfw_worker_destroy(w);
   __atomic_store_n(&hdr->worker_closed, session, __ATOMIC_RELEASE);
 }
 
@@ -572,14 +549,7 @@ int run_shm(const std::string& name, long mb, int device) {
     close(fd);
     return 4;
   }
-  std::memset(hdr, 0, sizeof *hdr);
-  hdr->version = TFSR_VERSION;
-  hdr->total_bytes = total;
-  tfsr_layout(total, &hdr->c2w_off, &hdr->c2w_size, &hdr->w2c_off, &hdr->w2c_size);
-  hdr->worker_pid = (uint32_t)getpid();
-  hdr->session = 1;
-  __atomic_store_n(&hdr->magic, TFSR_MAGIC, __ATOMIC_RELEASE);
-  __atomic_store_n(&hdr->worker_ready, 1u, __ATOMIC_RELEASE);
+  init_ring_header(hdr, total);
   printf("tensor-fusion-worker serving shmem %s (%ld MiB)\n", path.c_str(), mb);
   fflush(stdout);
   const char* once = getenv("TFW_ONESHOT");
@@ -588,7 +558,7 @@ int run_shm(const std::string& name, long mb, int device) {
     if (__atomic_load_n(&hdr->client_pid, __ATOMIC_ACQUIRE) == 0) { usleep(500); continue; }
     const uint32_t session = hdr->session;
     logf("client %u attached (session %u)", hdr->client_pid, session);
-    serve_shm_session(hdr, static_cast<uint8_t*>(m), total, device, session, fd, path);
+    serve_rings(hdr, static_cast<uint8_t*>(m), total, session, fd, path, make_worker(device));
     // next client: cursors keep counting (they are monotonic); whatever the last client left unread or
     // unsent is discarded while nobody is attached
     hdr->c2w_tail = __atomic_load_n(&hdr->c2w_head, __ATOMIC_ACQUIRE);
